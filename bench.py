@@ -46,6 +46,7 @@ LD_OUTPUTS = ["nd_map", "pd_map", "strong_nd_map", "weak_nd_map", "strong_pd_map
               "union_map_centralside"]
 DIGEST_OUTPUTS = LD_OUTPUTS + ["central_sess_high_dyn", "query_sess_high_dyn"]
 SIZES_PATH = os.path.join(ROOT, "tests", "golden", "config2_pass_sizes.json")
+DUMP_MAX_ROWS = 1 << 18                            # --dump-outputs: rows kept per output (4 MiB of float32 x 4), 40 MiB for all of DIGEST_OUTPUTS
 
 
 def schedule():
@@ -131,6 +132,14 @@ class ClockSampler:
         sm = [r[0] for r in self.rows]
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": float(self.max_sm), "reasons": sorted(reasons),
                 "samples": len(sm), "source": "nvml"}
+
+
+def dump_output(directory, name, a):
+    """Writes the (n, 4) float32 cloud `a` as directory/name.npy: all of it, or a seeded sample of DUMP_MAX_ROWS rows kept in order
+    (the outputs' point order is deterministic, so the same rows are compared between two builds)."""
+    if len(a) > DUMP_MAX_ROWS:
+        a = a[np.sort(np.random.default_rng(0).choice(len(a), DUMP_MAX_ROWS, replace=False))]
+    np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, np.float32))
 
 
 def owned_blocks(rank, world, kf, split):
@@ -352,6 +361,8 @@ def main():
     ap.add_argument("--no-split", action="store_true", help="every rank owns a block of BOTH sessions (no session split)")
     ap.add_argument("--no-e2e", action="store_true", help="diagnostic: skip the end-to-end arm")
     ap.add_argument("--no-clock-sampler", action="store_true", help="diagnostic: measure the sampler's own overhead")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the maps the last timed step produced as DIR/<name>.npy (float32, rank 0's "
+                    f"outputs, a seeded sample of {DUMP_MAX_ROWS} rows where larger)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -465,12 +476,17 @@ def main():
 
     # ---------------- digests of the step's outputs (parity across N: the driver's SCALE run must show identical ones) ----------------
     mine = {}
+    dump = args.dump_outputs if rank == 0 else None
+    if dump:
+        os.makedirs(dump, exist_ok=True)
     for name in DIGEST_OUTPUTS:
         try:
             a = R.cloud("saved:" + name)
         except Exception:  # noqa: BLE001 -- session-split: this rank does not hold that output
             continue
         mine[name] = [int(len(a)), hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()]
+        if dump:
+            dump_output(dump, name, a)
     allv = [None] * world
     if world > 1:
         dist.all_gather_object(allv, (mine, passlog))

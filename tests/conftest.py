@@ -14,9 +14,6 @@ def pytest_configure(config):
     # the native libraries are built artefacts (git-ignored): build them once if this checkout has none yet
     libs = [os.path.join(ROOT, "lt_mapper_b200", n) for n in ("libltr_b200.so", "libltr_removert.so", "ltremovert_b200")]
     libs += [os.path.join(ROOT, "oracle", "liboracle.so"), os.path.join(ROOT, "synth", "libltr_synth.so")]
-    if os.path.isdir("/root/reference/ltremovert/src"):     # the compiled-reference checker (oracle/ref_shim) can only be built where the reference is mounted
-        libs.append(os.path.join(ROOT, "oracle", "_ref", "libltremovert_ref.so"))
-        libs.append(os.path.join(ROOT, "oracle", "_ref", "libltremovert_dropin.so"))
     if not all(os.path.exists(p) for p in libs):
         import __graft_entry__
         __graft_entry__.build()

@@ -21,6 +21,8 @@ def _free_port():
 
 
 def _worker(rank, world, port, q):
+    # the buffers below are host memory: hide any GPU (before CUDA initialises) so that TorchDistComm takes its host path
+    os.environ["CUDA_VISIBLE_DEVICES"] = ""
     sys.path.insert(0, ROOT)
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)

@@ -6,7 +6,7 @@ import pytest
 
 from lt_mapper_b200 import removert
 
-REF_YAML = "/root/reference/ltremovert/config/params_ltmapper.yaml"
+REF_YAML = os.path.join(os.path.dirname(__file__), "golden", "params_ltmapper.yaml")      # the reference's shipped ltremovert/config/params_ltmapper.yaml
 
 
 def test_pcd_roundtrip_and_layout(tmp_path):
@@ -131,7 +131,6 @@ def test_yaml_reader(tmp_path):
     assert removert.yaml_get(p, "removert/dist_nn_points_within")[0] == "0.01"
 
 
-@pytest.mark.skipif(not os.path.exists(REF_YAML), reason="reference not mounted")
 def test_yaml_reader_on_the_reference_config():
     assert removert.yaml_get(REF_YAML, "removert/start_idx")[0] == "1100"
     assert removert.yaml_get(REF_YAML, "removert/keyframe_gap")[0] == "1"

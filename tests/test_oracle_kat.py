@@ -177,13 +177,17 @@ def test_knn_uses_squared_distances_and_exact_search():
     assert list(lab) == [1, 1]
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/ltslam/include/ltslam/nanoflann.hpp"), reason="reference not mounted")
 def test_kdtree_against_reference_nanoflann(tmp_path):
-    """Cross-check of the oracle's exact kNN against the reference's vendored nanoflann 1.3.2 (included by path, never copied)."""
+    """Cross-check of the oracle's exact kNN against the reference's vendored nanoflann 1.3.2 (included by path, never copied).  Its
+    distances are replayed from tests/golden/ref_nanoflann.json.gz (oracle/ref_golden.py); to record them from a checkout of the reference:
+    LTR_RECORD_REFERENCE=1 LTR_REFERENCE_DIR=<checkout> python -m pytest -p no:xdist tests/test_oracle_kat.py -k nanoflann"""
     import subprocess
+    from oracle.ref_golden import Recording, bits_equal
+    rec = Recording(os.path.join(os.path.dirname(__file__), "golden", "ref_nanoflann.json.gz"))
+    header = os.path.join(os.environ.get("LTR_REFERENCE_DIR", ""), "ltslam", "include", "ltslam", "nanoflann.hpp")
     src = tmp_path / "nf.cpp"
     src.write_text(r'''
-#include "/root/reference/ltslam/include/ltslam/nanoflann.hpp"
+#include NANOFLANN_HPP
 #include <cstdio>
 #include <vector>
 struct PC { std::vector<float> p; size_t kdtree_get_point_count() const { return p.size()/3; }
@@ -195,16 +199,21 @@ int main(int argc, char** argv) { FILE* f = fopen(argv[1], "rb"); int nt, nq, k;
   for (int i = 0; i < nq; ++i) { tree.knnSearch(&q[3*i], k, idx.data(), d.data()); fwrite(d.data(),4,k,o); } fclose(o); }
 ''')
     exe = tmp_path / "nf"
-    subprocess.check_call(["/usr/bin/g++", "-O2", "-ffp-contract=off", "-o", str(exe), str(src)])
     rng = np.random.default_rng(11)
     t = rng.uniform(-30, 30, (20000, 4)).astype(np.float32)
     q = rng.uniform(-30, 30, (2000, 4)).astype(np.float32)
     k = 3
-    with open(tmp_path / "in.bin", "wb") as f:
-        f.write(np.array([len(t), len(q), k], np.int32).tobytes()); f.write(t[:, :3].tobytes()); f.write(q[:, :3].tobytes())
-    subprocess.check_call([str(exe), str(tmp_path / "in.bin"), str(tmp_path / "out.bin")])
-    ref = np.fromfile(tmp_path / "out.bin", np.float32).reshape(len(q), k)
-    assert np.array_equal(ref.view(np.uint32), oracle.knn_dists(q, t, k).view(np.uint32))
+
+    def nanoflann():
+        subprocess.check_call(["/usr/bin/g++", "-O2", "-ffp-contract=off", f'-DNANOFLANN_HPP="{header}"', "-o", str(exe), str(src)])
+        with open(tmp_path / "in.bin", "wb") as f:
+            f.write(np.array([len(t), len(q), k], np.int32).tobytes()); f.write(t[:, :3].tobytes()); f.write(q[:, :3].tobytes())
+        subprocess.check_call([str(exe), str(tmp_path / "in.bin"), str(tmp_path / "out.bin")])
+        return np.fromfile(tmp_path / "out.bin", np.float32).reshape(len(q), k)
+    with rec.test("test_kdtree_against_reference_nanoflann"):
+        ref = rec.call("nanoflann knnSearch", (t, q, k), nanoflann)
+    rec.save()
+    assert bits_equal(ref, oracle.knn_dists(q, t, k))
 
 
 def test_faithful_mode_matches_exact_mode_single_thread(small_pair):

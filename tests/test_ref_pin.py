@@ -1,14 +1,14 @@
 """Pins the oracle (and the product's host-side file logic) against the reference's OWN code.
 
 oracle/_ref/libltremovert_ref.so holds ltremovert/src/{utility,RosParamServer,Session,Removerter}.cpp compiled unmodified
-from /root/reference against stand-in third-party headers (oracle/ref_shim/include/ltr_shim_core.h).  Every comparison is
+from the reference's sources against stand-in third-party headers (oracle/ref_shim/include/ltr_shim_core.h).  Every comparison is
 bit-exact.  What this pins: all first-party logic (projection, pixel indexing, min selection, discrepancy thresholds, index
 set arithmetic, kNN threshold test, schedule / run() order, keyframe parsing, pose reading).  What it does not: the
 third-party algorithms, whose stand-ins call the oracle's restatements (PCL transform / octree centroid / FLANN kNN / Eigen
 inverse).
 
-CPU only.  Skipped when oracle/_ref was not built (it is built by __graft_entry__.build() wherever /root/reference is mounted
-and travels to the GPU box as a prebuilt library).
+CPU only.  The reference's answers are replayed from tests/golden/ref_pin.json.gz (oracle/ref_golden.py), recorded from
+oracle/_ref where the reference's sources are available:  LTR_RECORD_REFERENCE=1 python -m pytest -p no:xdist tests/test_ref_pin.py
 """
 import os
 
@@ -16,17 +16,24 @@ import numpy as np
 import pytest
 
 import oracle
-from oracle import ref
+from oracle.ref_golden import RecordedRef, bits_equal, values_equal
 from lt_mapper_b200 import removert
 
-pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libltremovert_ref.so not built (needs /root/reference at build time)")
+ref = RecordedRef(os.path.join(os.path.dirname(__file__), "golden", "ref_pin.json.gz"))
 
 EXT = np.array([[np.cos(0.3), -np.sin(0.3), 0, 0.5], [np.sin(0.3), np.cos(0.3), 0, -0.2], [0, 0, 1, 1.1], [0, 0, 0, 1.0]])
 
 
-def bits_equal(a, b):
-    a = np.ascontiguousarray(a); b = np.ascontiguousarray(b)
-    return a.shape == b.shape and a.dtype == b.dtype and np.array_equal(a.view(np.uint8), b.view(np.uint8))
+@pytest.fixture(scope="module", autouse=True)
+def _save_recording(request):
+    yield
+    ref.rec.save(request.session.testsfailed == 0)
+
+
+@pytest.fixture(autouse=True)
+def _reference_calls(request):
+    with ref.rec.test(request.node.name):
+        yield
 
 
 def write_pcd(path, a):
@@ -83,11 +90,10 @@ def test_cart2sph_and_rad2deg_match_the_reference():
     p = _probe_points(np.random.default_rng(1))
     got = ref.cart2sph(p)
     x, y, z = p[:, 0], p[:, 1], p[:, 2]
-    assert bits_equal(got[:, 0], oracle.atan2f(y, x))
-    assert bits_equal(got[:, 1], oracle.atan2f(z, np.sqrt(x * x + y * y)))
-    assert bits_equal(got[:, 2], np.sqrt(x * x + y * y + z * z))
-    assert bits_equal(got[:, 2], oracle.pixel_index(p, 125, 900)[2])
-    a = np.concatenate([got[:, 0], got[:, 1]])
+    exp = np.stack([oracle.atan2f(y, x), oracle.atan2f(z, np.sqrt(x * x + y * y)), np.sqrt(x * x + y * y + z * z)], 1)
+    assert bits_equal(got, exp)
+    assert bits_equal(exp[:, 2], oracle.pixel_index(p, 125, 900)[2])
+    a = np.concatenate([exp[:, 0], exp[:, 1]])
     assert bits_equal(ref.rad2deg(a), (a.astype(np.float64) * 180.0 / np.pi).astype(np.float32))
 
 
@@ -133,13 +139,13 @@ def test_global_to_local_and_projected_parse_match_the_reference(small_pair, sma
 def test_index_set_arithmetic_matches_the_reference(scratch):
     # linspace<int>(0, N, N) (utility.h:158-167): integer step N / (N - 1) == 1 for N >= 3 -> 0 .. N-1
     for n in (3, 4, 17, 1000):
-        assert np.array_equal(ref.linspace_int(0, n, n), np.arange(n))
-    assert np.array_equal(ref.linspace_int(0, 2, 2), [0, 2])      # the N == 2 quirk the oracle / product document (index 2 is out of range)
+        assert values_equal(ref.linspace_int(0, n, n), np.arange(n))
+    assert values_equal(ref.linspace_int(0, 2, 2), [0, 2])      # the N == 2 quirk the oracle / product document (index 2 is out of range)
     R = ref.Removerter(base_params(scratch), write_files=False)
     rng = np.random.default_rng(3)
     for n in (3, 50, 5000):
         dyn = np.unique(rng.integers(0, n, n // 3)).astype(np.int32)
-        assert np.array_equal(R.static_idx(dyn, n), np.setdiff1d(np.arange(n), dyn))
+        assert values_equal(R.static_idx(dyn, n), np.setdiff1d(np.arange(n), dyn))
     R.close()
 
 
@@ -158,7 +164,7 @@ def test_remove_nd_pd_passes_match_the_reference(small_pair, small_maps, scratch
         R.set_cloud("map_global_curr_", m, 0)
         got = R.dynamic_idx(0, 0, 0, rows, cols, len(m))
         exp = oracle.remove_pass(m, c.xyzi, c.offsets, inv[0], oracle.MODE_HD, alpha, 0.1, lidar2base=l2b, order=order)
-        assert np.array_equal(got, np.flatnonzero(exp))
+        assert values_equal(got, np.flatnonzero(exp))
         assert len(got) > 100
     # ND (:485-540) and PD (:429-482) read the source session's keyframe_scans_static_projected_
     R.set_scans("keyframe_scans_static_projected_", q.xyzi, q.offsets, 1)
@@ -166,11 +172,11 @@ def test_remove_nd_pd_passes_match_the_reference(small_pair, small_maps, scratch
     R.set_cloud("map_global_nd_", m, 0)
     got = R.dynamic_idx(1, 0, 1, rows, cols, len(m))
     exp = oracle.remove_pass(m, q.xyzi, q.offsets, inv[1], oracle.MODE_ND, 2.5, 0.1, lidar2base=l2b, order=order)
-    assert np.array_equal(got, np.flatnonzero(exp)) and len(got) > 10
+    assert values_equal(got, np.flatnonzero(exp)) and len(got) > 10
     R.set_cloud("map_global_pd_", m, 0)
     got = R.dynamic_idx(2, 0, 1, rows, cols, len(m))
     exp = oracle.remove_pass(m, q.xyzi, q.offsets, inv[1], oracle.MODE_PD, 2.5, 0.1, lidar2base=l2b, order=order)
-    assert np.array_equal(got, np.flatnonzero(exp)) and len(got) > 10
+    assert values_equal(got, np.flatnonzero(exp)) and len(got) > 10
     R.close()
 
 
@@ -191,9 +197,10 @@ SAVED = ["OriginalNoisyCentralMapGlobal", "OriginalNoisyQueryMapGlobal", "centra
          "union_map_centralside", "pd_map", "nd_map", "strong_nd_map", "weak_nd_map", "strong_pd_map", "weak_pd_map", "updated_map", "updated_map_strong"]
 
 
-def _load_oracle_from_ref(R, O):
+def _load_oracle_from_ref(R, O, scans):
+    """scans[s]: the keyframe scans the reference loaded for session s (checked equal to R.scans("keyframe_scans_", s) by the caller)."""
     for s in (0, 1):
-        sc = R.scans("keyframe_scans_", s)
+        sc = scans[s]
         P, IP = R.keyframe_poses(s)
         off = np.concatenate([[0], np.cumsum([len(a) for a in sc])]).astype(np.int64)
         O.load_session(s, np.concatenate(sc), off, P, IP)
@@ -207,13 +214,15 @@ def test_run_matches_the_reference_stage_by_stage(session_files, small_pair, ord
         R.stage(st)
     assert R.num_keyframes(0) == small_pair[0].K and R.num_keyframes(1) == small_pair[1].K
     # file reading + pcl::VoxelGrid of Session::loadKeyframes against the product's host helpers
+    loaded = []
     for s in (0, 1):
         P, IP = R.keyframe_poses(s)
         assert bits_equal(P, removert.read_poses(f"{root}/{'central' if s == 0 else 'query'}/poses.txt"))
-        for k, a in enumerate(R.scans("keyframe_scans_", s)):
-            assert bits_equal(a, removert.voxel_grid(small_pair[s].scan(k), 0.05)[0])
+        got = R.scans("keyframe_scans_", s)
+        loaded.append([removert.voxel_grid(small_pair[s].scan(k), 0.05)[0] for k in range(small_pair[s].K)])
+        assert len(got) == len(loaded[s]) and all(bits_equal(a, b) for a, b in zip(got, loaded[s]))
     O = oracle.Removerter(num_knn=knn, knn_thr=thr, voxel=0.05, order=order, lidar2base=l2b, threads=4)
-    _load_oracle_from_ref(R, O)
+    _load_oracle_from_ref(R, O, loaded)
     for st, (clouds, scansets) in CLOUDS_AFTER.items():
         R.stage(st)
         O.stage(st)
@@ -237,7 +246,8 @@ def test_run_matches_the_reference_stage_by_stage(session_files, small_pair, ord
                         ("scans_pd", "keyframe_scans_pd_"), ("scans_pd_strong", "keyframe_scans_strong_pd_"), ("scans_nd_strong", "keyframe_scans_strong_nd_")):
         exp = O.clouds(member, 0)
         for k, nm in enumerate(names):
-            assert bits_equal(removert.read_pcd(f"{root}/out/{sub}/{nm}"), exp[k]), (sub, nm)
+            written = ref.capture("file written", (sub, nm), lambda: removert.read_pcd(f"{root}/out/{sub}/{nm}"))
+            assert bits_equal(written, exp[k]), (sub, nm)
     R.close()
 
 
@@ -260,7 +270,8 @@ def test_multi_resolution_schedules_match_the_reference(small_pair, scratch):
     for name in ("map_global_curr_", "map_global_curr_static_", "map_global_curr_dynamic_"):
         assert bits_equal(R.cloud(name, 0), O.cloud(name, 0)), name
     # the schedule bench.py runs: removeOnce at 2.5, 2.0, 1.5, then one revert at 1.0
-    R.set_cloud("map_global_curr_", m0, 0); R.set_cloud("map_global_curr_static_", m0[:0], 0); R.set_cloud("map_global_curr_dynamic_", m0[:0], 0)
+    none = np.zeros((0, 4), np.float32)
+    R.set_cloud("map_global_curr_", m0, 0); R.set_cloud("map_global_curr_static_", none, 0); R.set_cloud("map_global_curr_dynamic_", none, 0)
     for res in (2.5, 2.0, 1.5):
         R.op("removeOnce", 0, 0, res)
     R.op("resetAsDynamic", 0); R.op("revertOnce", 0, 0, 1.0); R.op("resetAsStatic", 0)
@@ -328,7 +339,7 @@ def test_non_default_fov_matches_the_reference(small_pair, small_maps, scratch, 
         R.set_cloud("map_global_curr_", m, 0)
         got = R.dynamic_idx(0, 0, 0, rows, cols, len(m))
         exp = oracle.remove_pass(m, c.xyzi, c.offsets, inv, oracle.MODE_HD, alpha, 0.1, vfov=vfov, hfov=hfov)
-        assert np.array_equal(got, np.flatnonzero(exp)) and len(got) > 100
+        assert values_equal(got, np.flatnonzero(exp)) and len(got) > 100
     R.close()
 
 
@@ -364,8 +375,6 @@ def test_property_random_clouds_match_the_reference():
     coord = st.one_of(f32, special)
     pts = st.lists(st.tuples(coord, coord, coord), min_size=1, max_size=200)
 
-    @settings(max_examples=60, deadline=None, suppress_health_check=list(HealthCheck))
-    @given(pts, st.sampled_from([0.1, 0.4, 2.5, 3.0]), st.booleans())
     def check(p, alpha, dup):
         a = np.array(p, np.float32).reshape(-1, 3)
         if dup:
@@ -374,9 +383,7 @@ def test_property_random_clouds_match_the_reference():
         got = ref.cart2sph(a)
         x, y, z = a[:, 0], a[:, 1], a[:, 2]
         with np.errstate(all="ignore"):
-            assert bits_equal(got[:, 0], oracle.atan2f(y, x))
-            assert bits_equal(got[:, 1], oracle.atan2f(z, np.sqrt(x * x + y * y)))
-            assert bits_equal(got[:, 2], np.sqrt(x * x + y * y + z * z))
+            assert bits_equal(got, np.stack([oracle.atan2f(y, x), oracle.atan2f(z, np.sqrt(x * x + y * y)), np.sqrt(x * x + y * y + z * z)], 1))
         rows, cols = oracle.reset_rimg_size(alpha)
         er, ei = oracle.map2rimg(cloud, rows, cols)
         gr, gi = ref.map2rimg(cloud, rows, cols)
@@ -386,7 +393,8 @@ def test_property_random_clouds_match_the_reference():
         exp, idx = oracle.parse_projected(cloud, np.eye(4), alpha)
         loc = ref.transform_global_to_local(cloud, np.eye(4), np.eye(4))   # as Session::parseScansViaProjection does (turns -0.0 into +0.0)
         assert bits_equal(ref.parse_projected(loc, rows, cols), exp) and 0 not in idx
-    check()
+    ref.rec.examples(check, lambda f: settings(max_examples=60, deadline=None, suppress_health_check=list(HealthCheck))(
+        given(pts, st.sampled_from([0.1, 0.4, 2.5, 3.0]), st.booleans())(f)))
 
 
 def test_property_random_passes_match_the_reference(scratch):
@@ -395,8 +403,6 @@ def test_property_random_passes_match_the_reference(scratch):
     from hypothesis import given, settings, strategies as st, HealthCheck
     R = ref.Removerter(base_params(scratch), write_files=False)
 
-    @settings(max_examples=40, deadline=None, suppress_health_check=list(HealthCheck))
-    @given(st.integers(0, 2**31 - 1), st.integers(3, 400), st.sampled_from([0.2, 0.5, 1.0, 2.5]), st.sampled_from([0, 1, 2]), st.booleans())
     def check(seed, n, alpha, mode, ties):
         rng = np.random.default_rng(seed)
         m = np.concatenate([rng.normal(0, 15, (n, 3)), rng.uniform(0, 1, (n, 1))], 1).astype(np.float32)
@@ -421,8 +427,9 @@ def test_property_random_passes_match_the_reference(scratch):
         R.set_cloud(["map_global_curr_", "map_global_nd_", "map_global_pd_"][mode], m, 0)
         got = R.dynamic_idx(mode, 0, 1 if mode else 0, rows, cols, len(m))
         exp = oracle.remove_pass(m, xyzi, off, inv, [oracle.MODE_HD, oracle.MODE_ND, oracle.MODE_PD][mode], alpha, 0.1)
-        assert np.array_equal(got, np.flatnonzero(exp))
-    check()
+        assert values_equal(got, np.flatnonzero(exp))
+    ref.rec.examples(check, lambda f: settings(max_examples=40, deadline=None, suppress_health_check=list(HealthCheck))(
+        given(st.integers(0, 2**31 - 1), st.integers(3, 400), st.sampled_from([0.2, 0.5, 1.0, 2.5]), st.sampled_from([0, 1, 2]), st.booleans())(f)))
     R.close()
 
 
@@ -432,8 +439,6 @@ def test_property_knn_partition_matches_the_reference(scratch):
     the squared-distance mean, the double accumulate, the strict threshold and the base2lidar matrix the reference passes to local2global)."""
     from hypothesis import given, settings, strategies as st, HealthCheck
 
-    @settings(max_examples=25, deadline=None, suppress_health_check=list(HealthCheck))
-    @given(st.integers(0, 2**31 - 1), st.sampled_from([1, 2, 3]), st.sampled_from([0.01, 0.04, 0.5, 4.0]), st.booleans(), st.booleans(), st.sampled_from([0, 1]))
     def check(seed, k, thr, low, use_ext, order):
         rng = np.random.default_rng(seed)
         l2b = EXT if use_ext else np.eye(4)
@@ -468,7 +473,9 @@ def test_property_knn_partition_matches_the_reference(scratch):
             if co is not None:
                 assert bits_equal(co[j], eco), (j, "coexist")
         R.close()
-    check()
+    ref.rec.examples(check, lambda f: settings(max_examples=25, deadline=None, suppress_health_check=list(HealthCheck))(
+        given(st.integers(0, 2**31 - 1), st.sampled_from([1, 2, 3]), st.sampled_from([0.01, 0.04, 0.5, 4.0]), st.booleans(), st.booleans(),
+              st.sampled_from([0, 1]))(f)))
 
 
 def test_property_keyframe_selection_and_pose_files_match_the_reference(tmp_path_factory, scratch):
@@ -478,8 +485,6 @@ def test_property_keyframe_selection_and_pose_files_match_the_reference(tmp_path
     from hypothesis import given, settings, strategies as st, HealthCheck
     counter = [0]
 
-    @settings(max_examples=40, deadline=None, suppress_health_check=list(HealthCheck))
-    @given(st.integers(0, 2**31 - 1), st.integers(1, 40), st.integers(1, 40), st.integers(-3, 45), st.integers(-3, 45), st.integers(1, 7))
     def check(seed, nc, nq, start, end, gap):
         rng = np.random.default_rng(seed)
         counter[0] += 1
@@ -502,12 +507,13 @@ def test_property_keyframe_selection_and_pose_files_match_the_reference(tmp_path
         assert bits_equal(pc, poses["central"]) and bits_equal(pq, poses["query"])
         exp_c = list(removert.parse_keyframes(nc, start, end, gap))
         assert R.keyframe_names(0) == [f"{k:06d}.pcd" for k in exp_c]
-        kc = R.keyframe_poses(0)[0]
-        assert bits_equal(kc, pc[exp_c].reshape(-1, 4, 4))
+        kc = pc[exp_c].reshape(-1, 4, 4)
+        assert bits_equal(R.keyframe_poses(0)[0], kc)
         exp_q = list(removert.parse_keyframes_in_roi(pq, kc, gap))
         assert R.keyframe_names(1) == [f"{k:06d}.pcd" for k in exp_q]
         R.close()
-    check()
+    ref.rec.examples(check, lambda f: settings(max_examples=40, deadline=None, suppress_health_check=list(HealthCheck))(
+        given(st.integers(0, 2**31 - 1), st.integers(1, 40), st.integers(1, 40), st.integers(-3, 45), st.integers(-3, 45), st.integers(1, 7))(f)))
 
 
 def test_points_on_pixel_boundaries_land_in_the_reference_pixel():
@@ -534,15 +540,19 @@ def test_points_on_pixel_boundaries_land_in_the_reference_pixel():
         pts = np.array(pts, np.float32)
         er, ec, erng = oracle.pixel_index(pts, rows, cols, vfov, hfov)
         first = np.array([[1.0, 0.0, 0.0, 0.0]], np.float32)     # index 0 is "no point" in the index image: keep a dummy there
-        moved = 0
-        for i, p in enumerate(pts):
-            cloud = np.concatenate([first * 1e3, np.concatenate([p, [0.0]]).astype(np.float32)[None]])   # dummy far away at az = el = 0
-            gr, gi = ref.map2rimg(cloud, rows, cols, vfov, hfov)
-            rr, cc = np.argwhere(gi == 1)[0] if (gi == 1).any() else (-1, -1)
-            assert (rr, cc) == (er[i], ec[i]), (i, p, (rr, cc), (er[i], ec[i]))
-            assert gr[rr, cc].view(np.uint32) == erng[i].view(np.uint32)
-            moved += 1
-        assert moved == count
+
+        def landings():
+            """Per point: (row, col, range bits) where the reference's map2RangeImg puts it."""
+            out = []
+            for p in pts:
+                cloud = np.concatenate([first * 1e3, np.concatenate([p, [0.0]]).astype(np.float32)[None]])   # dummy far away at az = el = 0
+                gr, gi = ref.compiled.map2rimg(cloud, rows, cols, vfov, hfov)
+                rr, cc = np.argwhere(gi == 1)[0] if (gi == 1).any() else (-1, -1)
+                out.append((rr, cc, gr[rr, cc].view(np.uint32)))
+            return np.array(out, np.int64)
+        got = ref.capture("map2rimg landings", (pts, rows, cols, vfov, hfov), landings)
+        assert len(got) == count
+        assert values_equal(got, np.stack([er, ec, erng.view(np.uint32)], 1).astype(np.int64))
 
 
 def test_full_size_scans_match_the_reference(scratch):
